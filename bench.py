@@ -3,12 +3,13 @@
 
 One "step" = one pass of the hot path (decode every block of the shard) over synthetic input.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--gib G]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--gib G] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): seekable ZXC frame, 64 KiB blocks, level 3, over the
 Silesia-shaped synthetic corpus (oracle/zxc_corpus.c), G GiB decoded per GPU (default 4; 8 at N = 8 = configs[4]'s 64 GiB).
-Frames are produced by the UNMODIFIED reference encoder (oracle/_ref, see BASELINE.md section 3);
-at N > 1 every rank owns the contiguous block range [rank*G GiB, (rank+1)*G GiB) of the frame
+Frames are produced by this library's GPU encoder, whose frames are byte-identical to the reference
+encoder's (BASELINE.md section 3): for the default inputs the frame's sha256 is checked against the reference's
+(tests/golden/bench/reference.json) before anything is timed.  At N > 1 every rank owns the contiguous block range [rank*G GiB, (rank+1)*G GiB) of the frame
 (weak scaling: independent seekable blocks, no data-path collective).
 
   value        decode-only, compressed input and output resident in HBM, CUDA events on the
@@ -20,8 +21,9 @@ at N > 1 every rank owns the contiguous block range [rank*G GiB, (rank+1)*G GiB)
   e2e_pageable the same call with ordinary (pageable) numpy buffers: the library stages them through its own
                NUMA-local pinned bounce buffers and copy pools.
   cpu_baseline the reference's own SIMD CPU path (zxc_seekable_decompress_range_mt, all host
-               threads; zxc_decompress 1 thread) on the same frame, same run, rank 0 at N=1.
-  dict         (N=1) BASELINE configs[3]: trained dictionary, 1 Mi x 4 KiB records, level 5, one frame with
+               threads; zxc_decompress 1 thread) on the same frame, same run, rank 0 at N=1; only where
+               the reference library was built (oracle/_ref), otherwise reported as not measured.
+  dict         (N=1) BASELINE configs[3]: the reference trainer's dictionary (tests/golden/bench/records_dict.bin), 1 Mi x 4 KiB records, level 5, one frame with
                block_size 4096 -- decode-only value + roofline, e2e through zxc_seekable_set_dict +
                zxc_seekable_decompress_range_mt, the reference's CPU figure for the same calls.
   encode       (N=1) BASELINE configs[2]: level 6 over 1 GiB through zxc_compress, frame compared with the reference's.
@@ -29,7 +31,10 @@ at N > 1 every rank owns the contiguous block range [rank*G GiB, (rank+1)*G GiB)
                NCCL scatter of compressed block ranges -> decode -> NCCL gather into rank 0, each phase timed on
                the device (max over ranks), output verified on rank 0.
   Every rank binds itself to its GPU's NUMA node before it allocates pinned host memory.
-  --impl reference   times only that CPU path, same metric / config.
+  --impl reference   times only that CPU path, same metric / config (needs oracle/_ref).
+  --dump-outputs DIR after the timed steps, rank 0 writes what the last timed step computed as DIR/<name>.npy:
+               block_status (per-block result of zxc_b200_decode_blocks), block_sums (per-block byte sums of the
+               decoded output) and decoded_sample (decoded bytes at 8 Mi fixed, seeded positions), float64 / float32.
 """
 import argparse
 import ctypes as C
@@ -48,6 +53,14 @@ import numpy as np  # noqa: E402
 
 BLOCK = 65536
 LEVEL = 3
+DEFAULT_GIB = 4.0
+ENCODE_BYTES = 1 << 30  # input of the encode leg: the first GiB of rank 0's shard
+DICT_REC = 4096
+DICT_RECORDS = 1 << 20
+DICT_TRAIN_SAMPLES = 4096  # the stored dictionary was trained on the first 4096 records
+DICT_IDENTITY_RECORDS = 2048
+DUMP_SAMPLE = 1 << 23
+GOLDEN = os.path.join(ROOT, "tests", "golden", "bench")
 
 
 class Job(C.Structure):
@@ -173,17 +186,49 @@ class ClockSampler:
                 "samples": len(sm), "source": "nvml" if self.nvml is not None else "nvidia-smi"}
 
 
-def build_shard(ref, gib, rank, seed=1):
-    """(data ndarray, frame ndarray) for this rank's slice of the Silesia-shaped stream."""
+def shard_input(gib, rank, seed=1):
+    """this rank's slice of the Silesia-shaped stream"""
     import zxc_corpus as zc
     n = int(gib * (1 << 30))
     n -= n % (1 << 20)
+    return zc.silesia_shaped(n, seed=seed, offset=rank * n)
+
+
+def frame_key(gib, rank, level):
+    return f"frame_gib{gib:g}_rank{rank}_level{level}"
+
+
+def sha256(a):
+    import hashlib
+    return hashlib.sha256(memoryview(np.ascontiguousarray(a))).hexdigest()
+
+
+def reference_sha(key):
+    """sha256 of the reference encoder's frame for `key`, or None when none is stored"""
+    return json.load(open(os.path.join(GOLDEN, "reference.json"))).get(key)
+
+
+def build_shard(lib, gib, rank, on_gpu):
+    """(data ndarray, frame ndarray) for this rank's slice; the frame from `lib`'s encoder (one 1 GiB call after the
+    other on the GPU, parallel slices on the CPU) stitched into one seekable frame, and checked against the
+    reference's frame where its sha256 is stored."""
+    import zxc_corpus as zc
     t0 = time.time()
-    data = zc.silesia_shaped(n, seed=seed, offset=rank * n)
+    data = shard_input(gib, rank)
     t1 = time.time()
-    frame = zc.compress_ref_mt(ref, data, level=LEVEL, block_size=BLOCK, checksum=0)
+    kw = {"threads": 1, "slice_bytes": min(1 << 30, data.size)} if on_gpu else {}
+    frame = zc.compress_ref_mt(lib, data, level=LEVEL, block_size=BLOCK, checksum=0, **kw)
     t2 = time.time()
-    return data, frame, {"gen_s": round(t1 - t0, 2), "ref_compress_s": round(t2 - t1, 2)}
+    want = reference_sha(frame_key(gib, rank, LEVEL))
+    identical = None if want is None else sha256(frame) == want
+    assert identical is not False, "the frame differs from the reference encoder's frame"
+    return data, frame, {"gen_s": round(t1 - t0, 2), "compress_s": round(t2 - t1, 2),
+                         "frame_identical_to_reference": identical}
+
+
+def load_ref():
+    import zxc_ctypes as z
+    return z.ZxcLib(z.REF_SO) if z.have_ref() else None
 
 
 def cpu_reference_decode(ref, frame, n, threads, reps):
@@ -330,21 +375,21 @@ def pipeline_leg(lib, dist, dev, stream, rank, world, frame, jv, data, steps, bl
 
 
 def dict_leg(lib, prod, ref, dev, stream, threads, n_records, steps, peak):
-    """BASELINE.json configs[3]: 16 KiB dictionary (the reference's trainer), n x 4 KiB records, level 5, one
-    seekable frame with block_size 4096.  value = decode-only from HBM; e2e = zxc_seekable_set_dict +
-    zxc_seekable_decompress_range_mt of THIS library with host buffers; cpu = the same two calls of the reference."""
+    """BASELINE.json configs[3]: 16 KiB dictionary (the reference's trainer over the first 4096 records, stored in
+    tests/golden/bench/records_dict.bin), n x 4 KiB records, level 5, one seekable frame with block_size 4096.
+    value = decode-only from HBM; e2e = zxc_seekable_set_dict + zxc_seekable_decompress_range_mt of THIS library
+    with host buffers; cpu = the same two calls of the reference, where it was built."""
     import torch
     import zxc_corpus as zc
-    import zxc_ctypes as z
-    REC = 4096
+    REC = DICT_REC
+    assert n_records >= DICT_TRAIN_SAMPLES, f"--dict-records must be at least {DICT_TRAIN_SAMPLES}"
     data = zc.records(n_records, REC)
-    dict_bytes = zc.train_dict_ref(ref, data, REC)
+    dict_bytes = open(os.path.join(GOLDEN, "records_dict.bin"), "rb").read()
     dsz = len(dict_bytes)
     frame = prod.compress(data, level=5, block_size=REC, seekable=1, dict=dict_bytes)  # GPU encoder
     assert not isinstance(frame, int), frame
-    sub = data[: 2048 * REC]
-    identical = bool(np.array_equal(ref.compress(sub, level=5, block_size=REC, seekable=1, dict=dict_bytes),
-                                    prod.compress(sub, level=5, block_size=REC, seekable=1, dict=dict_bytes)))
+    sub = data[: DICT_IDENTITY_RECORDS * REC]
+    identical = sha256(prod.compress(sub, level=5, block_size=REC, seekable=1, dict=dict_bytes)) == reference_sha("dict_level5")
     n = data.size
     nb = lib.zxc_b200_plan_frame(frame.ctypes.data, frame.size, None, 0, None)
     jobs = np.zeros(nb * C.sizeof(Job), dtype=np.uint8)
@@ -395,9 +440,11 @@ def dict_leg(lib, prod, ref, dev, stream, threads, n_records, steps, peak):
         return n / best / 1e9
     e2e = seek_run(prod.lib, h_frame.data_ptr(), h_frame.numel(), h_out.data_ptr(), 3)
     assert np.array_equal(h_out.numpy(), data), "dict leg: e2e output differs"
-    out = np.zeros(n, dtype=np.uint8)
-    cpu = seek_run(ref.lib, frame.ctypes.data, frame.size, out.ctypes.data, 3)
-    assert np.array_equal(out, data)
+    cpu = None
+    if ref is not None:
+        out = np.zeros(n, dtype=np.uint8)
+        cpu = round(seek_run(ref.lib, frame.ctypes.data, frame.size, out.ctypes.data, 3), 3)
+        assert np.array_equal(out, data)
     achieved = (comp_bytes + n) / (ms * 1e-3) / 1e9
     return {"workload": f"zxc_dict decode: {dsz} B dictionary (reference trainer), {n_records} x 4 KiB records, level 5, "
                         "block_size 4096, one seekable frame",
@@ -408,8 +455,26 @@ def dict_leg(lib, prod, ref, dev, stream, threads, n_records, steps, peak):
                          "note": "C + U per record; the dictionary is read once per SM and excluded (SURVEY 8(d))"},
             "e2e": {"value": round(e2e, 2), "unit": "GB/s", "h2d_bytes_per_step": int(frame.size), "d2h_bytes_per_step": int(n),
                     "api": "zxc_seekable_open + zxc_seekable_set_dict + zxc_seekable_decompress_range_mt, pinned host buffers"},
-            "cpu_baseline": {"value": round(cpu, 3), "unit": "GB/s", "cores": threads, "kind": "reference",
-                             "sample": "the same frame, zxc_seekable_set_dict + zxc_seekable_decompress_range_mt, best of 3"}}
+            "cpu_baseline": {"value": cpu, "unit": "GB/s", "cores": threads, "kind": "reference",
+                             "sample": "the same frame, zxc_seekable_set_dict + zxc_seekable_decompress_range_mt, best of 3"
+                                       if cpu is not None else "not measured: reference library not built (oracle/_ref)"}}
+
+
+def dump_outputs(out_dir, d_dst, d_status):
+    """what the last timed step left in HBM: the per-block verdicts, per-block byte sums of the decoded output and the
+    decoded bytes at DUMP_SAMPLE positions drawn with a fixed seed (the whole output is GiBs)"""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = d_dst.numel()
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    sample = d_dst[torch.from_numpy(idx).to(d_dst.device)].cpu().numpy()
+    np.save(os.path.join(out_dir, "decoded_sample.npy"), sample.astype(np.float32))
+    nfull = n - n % BLOCK
+    sums = d_dst[:nfull].view(-1, BLOCK).sum(dim=1, dtype=torch.int64).cpu().numpy()
+    if nfull < n:
+        sums = np.append(sums, int(d_dst[nfull:].sum(dtype=torch.int64)))
+    np.save(os.path.join(out_dir, "block_sums.npy"), sums.astype(np.float64))
+    np.save(os.path.join(out_dir, "block_status.npy"), d_status.cpu().numpy().astype(np.float64))
 
 
 def main():
@@ -422,22 +487,21 @@ def main():
                     "GPUs hold configs[4]'s 64 GiB frame)")
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--decode-only", action="store_true", help="development: skip the cpu_baseline, dict and encode legs")
-    ap.add_argument("--dict-records", type=int, default=1 << 20, help="records of the configs[3] dictionary leg")
+    ap.add_argument("--dict-records", type=int, default=DICT_RECORDS, help="records of the configs[3] dictionary leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.gib <= 0:
-        args.gib = 8.0 if world >= 8 else 4.0
+        args.gib = 8.0 if world >= 8 else DEFAULT_GIB
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
 
     import zxc_corpus as zc
     import zxc_ctypes as z
 
-    if not os.path.exists(z.REF_SO):
-        raise SystemExit("oracle/_ref/libzxc_ref.so missing: run __graft_entry__.build() where /root/reference exists")
-    ref = z.ZxcLib(z.REF_SO)
+    ref = load_ref()
     threads = zc.host_threads()
     config = {"workload": f"seekable decode, {args.gib:g} GiB/GPU Silesia-shaped synthetic, 64 KiB blocks, level 3",
               "block_size": BLOCK, "level": LEVEL, "gib_per_gpu": args.gib, "sharding": f"block-range x{world}",
@@ -447,7 +511,9 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        data, frame, prep = build_shard(ref, args.gib, 0)
+        if ref is None:
+            raise SystemExit("--impl reference needs oracle/_ref/libzxc_ref.so: build() compiles it where the reference sources are")
+        data, frame, prep = build_shard(ref, args.gib, 0, on_gpu=False)
         n = data.size
         out = np.zeros(n, dtype=np.uint8)
         h = ref.lib.zxc_seekable_open(frame.ctypes.data, frame.size)
@@ -496,7 +562,7 @@ def main():
     lib.zxc_b200_reduce_status.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]
     lib.zxc_b200_launch_count.restype = C.c_uint64
 
-    data, frame, prep = build_shard(ref, args.gib, rank)
+    data, frame, prep = build_shard(prod, args.gib, rank, on_gpu=True)
     n = data.size
     info = Info()
     nb = lib.zxc_b200_plan_frame(frame.ctypes.data, frame.size, None, 0, C.byref(info))
@@ -554,6 +620,8 @@ def main():
     total_ms = evs[0].elapsed_time(evs[-1])
     per_launch_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_dst, d_status)
 
     t_ms = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -563,7 +631,7 @@ def main():
 
     # ---- e2e through the C ABI with host (pinned) buffers: H2D + decode + D2H every step
     h_out = torch.empty(n, dtype=torch.uint8).pin_memory()
-    e2e_steps = max(2, min(args.steps, 5))
+    e2e_steps = args.steps
     for _ in range(2):
         r = prod.lib.zxc_decompress(h_frame.data_ptr(), h_frame.numel(), h_out.data_ptr(), n, None)
         assert r == n, r
@@ -590,9 +658,9 @@ def main():
     if world > 1:
         dist.barrier()
     t0 = time.perf_counter()
-    for _ in range(2):
+    for _ in range(args.steps):
         r = prod.lib.zxc_decompress(frame.ctypes.data, frame.size, p_out.ctypes.data, n, None)
-    pg_dt = (time.perf_counter() - t0) / 2
+    pg_dt = (time.perf_counter() - t0) / args.steps
     assert r == n
     if not args.no_verify:
         assert np.array_equal(p_out, data), "pageable e2e output differs"
@@ -673,7 +741,7 @@ def main():
     if world > 1:
         del d_scratch
         torch.cuda.empty_cache()
-        pipeline = pipeline_leg(lib, dist, dev, stream, rank, world, frame, jv, data, max(2, min(args.steps, 5)), BLOCK)
+        pipeline = pipeline_leg(lib, dist, dev, stream, rank, world, frame, jv, data, args.steps, BLOCK)
 
     if rank == 0:
         peak, peak_src = measured_peak()
@@ -710,20 +778,24 @@ def main():
             os.sched_setaffinity(0, all_cpus)  # the CPU baseline may use every host core again
             threads = zc.host_threads()
             reps = 3
-            mt, out = cpu_reference_decode(ref, frame, n, threads, reps)
-            sample_n = min(n, 256 << 20)
-            sf = zc.compress_ref_mt(ref, data[:sample_n], level=LEVEL, block_size=BLOCK)
-            o1 = np.zeros(sample_n, dtype=np.uint8)
-            t = time.perf_counter()
-            r1 = ref.lib.zxc_decompress(sf.ctypes.data, sf.size, o1.ctypes.data, sample_n, None)
-            st = sample_n / (time.perf_counter() - t) / 1e9
-            assert r1 == sample_n
-            line["cpu_baseline"] = {"value": round(mt, 3), "unit": "GB/s", "cores": threads, "kind": "reference",
-                                    "sample": f"whole {args.gib:g} GiB frame, zxc_seekable_decompress_range_mt best of {reps}",
-                                    "single_thread_gbs": round(st, 3)}
+            if ref is not None:
+                mt, out = cpu_reference_decode(ref, frame, n, threads, reps)
+                sample_n = min(n, 256 << 20)
+                sf = zc.compress_ref_mt(ref, data[:sample_n], level=LEVEL, block_size=BLOCK)
+                o1 = np.zeros(sample_n, dtype=np.uint8)
+                t = time.perf_counter()
+                r1 = ref.lib.zxc_decompress(sf.ctypes.data, sf.size, o1.ctypes.data, sample_n, None)
+                st = sample_n / (time.perf_counter() - t) / 1e9
+                assert r1 == sample_n
+                line["cpu_baseline"] = {"value": round(mt, 3), "unit": "GB/s", "cores": threads, "kind": "reference",
+                                        "sample": f"whole {args.gib:g} GiB frame, zxc_seekable_decompress_range_mt best of {reps}",
+                                        "single_thread_gbs": round(st, 3)}
+            else:
+                line["cpu_baseline"] = {"value": None, "unit": "GB/s", "kind": "reference",
+                                        "sample": "not measured: reference library not built (oracle/_ref)"}
             # ---- supplementary: the encoder, BASELINE.json configs[2] (level 6, 1 GiB, frame bit-exact vs the
             # reference) and the same input at level 3; through zxc_compress with host buffers
-            enc_n = min(n, 1 << 30)
+            enc_n = min(n, ENCODE_BYTES)
             src_v = data[:enc_n]
             cap = int(prod.lib.zxc_compress_bound(enc_n))
             enc_out = np.zeros(cap, dtype=np.uint8)
@@ -734,17 +806,21 @@ def main():
                 t = time.perf_counter()
                 r_enc = prod.lib.zxc_compress(src_v.ctypes.data, enc_n, enc_out.ctypes.data, cap, C.byref(o))
                 enc_dt = time.perf_counter() - t
-                t = time.perf_counter()
-                ref_frame = zc.compress_ref_mt(ref, src_v, level=level, block_size=BLOCK)
-                ref_dt = time.perf_counter() - t
+                want = reference_sha(frame_key(enc_n / (1 << 30), 0, level))
+                cpu_gbs = None
+                if ref is not None:
+                    t = time.perf_counter()
+                    ref_frame = zc.compress_ref_mt(ref, src_v, level=level, block_size=BLOCK)
+                    cpu_gbs = round(enc_n / (time.perf_counter() - t) / 1e9, 3)
+                    want = sha256(ref_frame)
                 return {"level": level, "bytes_in": int(enc_n), "gbs_in_e2e": round(enc_n / enc_dt / 1e9, 3),
-                        "identical_to_reference": bool(r_enc == ref_frame.size and np.array_equal(enc_out[:r_enc], ref_frame)),
+                        "identical_to_reference": None if want is None else r_enc > 0 and sha256(enc_out[:r_enc]) == want,
                         "ratio": round(r_enc / enc_n, 4),
-                        "cpu_reference_gbs_in": round(enc_n / ref_dt / 1e9, 3), "cpu_threads": threads}
+                        "cpu_reference_gbs_in": cpu_gbs, "cpu_threads": threads}
 
             del d_src, d_dst
             torch.cuda.empty_cache()
-            line["dict"] = dict_leg(lib, prod, ref, dev, stream, threads, args.dict_records, max(3, args.steps), peak)
+            line["dict"] = dict_leg(lib, prod, ref, dev, stream, threads, args.dict_records, args.steps, peak)
             line["encode"] = encode_leg(6)
             line["encode"]["note"] = "configs[2]: optimal parser + Huffman sections on the GPU; levels 1-7 all encode on the GPU"
             line["encode"]["level3"] = encode_leg(LEVEL)

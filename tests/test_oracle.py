@@ -92,13 +92,21 @@ def test_oracle_golden_format_decode(orc):
     assert r == 16384 and int(o.max()) < 220
 
 
-def test_hashes_against_reference(orc, ref):
+def dict_id_cases():
+    """(n, content, huf128) triples, seeded"""
     rng = np.random.default_rng(7)
     for n in list(range(1, 40)) + [47, 48, 49, 111, 112, 113, 114, 223, 224, 225, 300, 4096, 65537]:
         b = rng.integers(0, 256, n, dtype=np.uint8).tobytes()
-        assert orc.lib.zxo_dict_id(b, n, None) == ref.lib.zxc_dict_id(b, n, None), n
         huf = rng.integers(0, 256, 128, dtype=np.uint8).tobytes()
-        assert orc.lib.zxo_dict_id(b, n, huf) == ref.lib.zxc_dict_id(b, n, huf), n
+        yield n, b, huf
+
+
+def test_hashes_against_reference(orc):
+    """zxc_dict_id of the reference for dict_id_cases(), without and with the Huffman table, is stored in
+    tests/golden/reference/dict_ids.json (tests/golden/make_fixtures.py)"""
+    want = json.load(open(os.path.join(G, "reference", "dict_ids.json")))
+    got = [[n, orc.lib.zxo_dict_id(b, n, None), orc.lib.zxo_dict_id(b, n, huf)] for n, b, huf in dict_id_cases()]
+    assert got == want
 
 
 CASES = [("silesia", 3 << 20), ("text", 300000), ("random", 70000), ("numeric", 200000),

@@ -94,8 +94,9 @@ def test_kernel_source_damaged_blocks_fail_like_the_reference(prod, ref):
         assert checked >= 40
 
 
-def test_kernel_source_differential_fuzz_smoke():
-    """a short fixed-seed run of the open-ended emulator fuzz tools (tests/simt_fuzz.py, tests/simt_fuzz_dict.py)"""
+def test_kernel_source_differential_fuzz_smoke(ref):
+    """a short fixed-seed run of the open-ended emulator fuzz tools (tests/simt_fuzz.py, tests/simt_fuzz_dict.py);
+    both draw their frames and verdicts from the reference library"""
     import subprocess
     import sys
     here = os.path.dirname(os.path.abspath(__file__))
