@@ -71,7 +71,25 @@ ZXC_EXPORT size_t zxc_b200_decode_scratch_size(uint32_t block_size);
  *   d_dict    dictionary content or NULL; d_dict_huf its 128-byte table or NULL
  *   d_scratch zxc_b200_decode_scratch_size(block_size) bytes
  *   verify_checksums  non-zero: jobs carry a trailing rapidhash fold, check it
- * Returns ZXC_OK once the launch is enqueued, or a negative code. */
+ * Returns ZXC_OK once the launch is enqueued, or a negative code: ZXC_ERROR_NULL_INPUT when d_src, d_dst, d_jobs,
+ * d_status or d_scratch is NULL; ZXC_ERROR_MEMORY when scratch_size is below what this launch needs (then nothing
+ * is launched and d_status is untouched).  n_jobs == 0 launches nothing.
+ *
+ * What a caller may rely on (tests/test_device_abi_gpu.py, tests/test_simt_layouts.py):
+ *   - no alignment is required of d_src, d_dst, d_dict, d_dict_huf or of any src_off / dst_off;
+ *   - offsets are full 64-bit byte offsets (buffers beyond 4 GiB);
+ *   - the job table is any list of jobs: any order, a subset of a frame's blocks with rebased offsets, gaps or
+ *     overlaps between source ranges, the same source block decoded to several windows.  Output windows
+ *     [dst_off, dst_off + dst_cap) of different jobs must not overlap;
+ *   - a job writes nothing outside its window, whatever its block holds.  Its status is what the reference's block
+ *     decoder gives for that block at that dst_cap, including DST_TOO_SMALL / OVERFLOW when dst_cap is too small;
+ *     its bytes are valid only where the status is >= 0, and only the first `status` of them;
+ *   - every job's dst_cap is at most block_size, which sizes the scratch (it need not be the frame's block size);
+ *   - d_dict_huf may live in an allocation of its own; it need not follow the dictionary;
+ *   - jobs without a dictionary reference ignore d_dict; a block that refers to one needs it;
+ *   - one scratch serves any number of launches in stream order without being cleared (its last 32 bytes hold the
+ *     launch's work counters, which every launch resets); launches that may run at the same time, on different
+ *     streams, each need their own scratch, status and output. */
 ZXC_EXPORT int zxc_b200_decode_blocks(const void* d_src, void* d_dst, const zxc_b200_job_t* d_jobs,
                                       uint32_t n_jobs, int32_t* d_status, const void* d_dict,
                                       uint32_t dict_size, const void* d_dict_huf, void* d_scratch,
@@ -79,9 +97,9 @@ ZXC_EXPORT int zxc_b200_decode_blocks(const void* d_src, void* d_dst, const zxc_
                                       int verify_checksums, void* stream);
 
 /* Reduce a status array (device) to the reference's frame verdict: total bytes
- * if every job produced exactly its dst_cap, else the first failing job's code
- * in stream order (ZXC_ERROR_CORRUPT_DATA for a size mismatch).  Synchronises
- * `stream`. */
+ * if every job produced exactly its dst_cap (a 64-bit sum), else the code of the
+ * failing job with the lowest index (ZXC_ERROR_CORRUPT_DATA for a size mismatch).
+ * 0 for n_jobs == 0.  Synchronises `stream`. */
 ZXC_EXPORT int64_t zxc_b200_reduce_status(const int32_t* d_status, const zxc_b200_job_t* d_jobs,
                                           uint32_t n_jobs, void* stream);
 

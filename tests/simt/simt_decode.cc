@@ -39,6 +39,7 @@ extern "C" uint64_t simt_decode_blocks(const u8* src, uint64_t src_size, u8* dst
     /* device buffers with a guard band either side: word loads may touch a few bytes outside, stores must not */
     std::vector<u8> in(src_size + 2 * PAD, 0xA5), out(dst_size + 2 * PAD, 0x5A), dct((size_t)dict_size + 128 + 2 * PAD, 0x33);
     memcpy(in.data() + PAD, src, src_size);
+    memcpy(out.data() + PAD, dst, dst_size); /* the caller's bytes: what a job does not write must come back unchanged */
     if (dict && dict_size) memcpy(dct.data() + PAD, dict, dict_size);
     if (dict_huf) memcpy(dct.data() + PAD + dict_size, dict_huf, 128);
     const u32 stride = scr_stride(block_cap);

@@ -1,6 +1,7 @@
 """TEST INFRASTRUCTURE: ctypes binding of tests/simt/libzxc_simt_decode.so -- the product's decode DEVICE code compiled
 for the CPU on the fiber warp emulator (tests/simt/).  decode_frame() plans a frame with the product's host code
-(zxc_b200_plan_frame, no device needed) and runs decode_job() once per block on an emulated warp."""
+(zxc_b200_plan_frame, no device needed) and runs decode_job() once per block on an emulated warp; decode_jobs() runs a
+caller-built job table the same way."""
 import ctypes as C
 import os
 import subprocess
@@ -58,7 +59,7 @@ def decode_frame(prod, frame, dict=None, dict_huf=None, verify=0, units=0, seed=
     if max_blocks is not None:
         nb = min(nb, max_blocks)
     total = int(jobs[nb - 1].dst_off + jobs[nb - 1].dst_cap) if nb else 0
-    out = np.zeros(max(total, 1), np.uint8)
+    out = np.full(max(total, 1), 0x5A, np.uint8)  # a byte no job writes reads back as 0x5A, not as a plausible 0
     status = (C.c_int32 * max(nb, 1))()
     oob = C.c_int(0)
     src = np.frombuffer(fb, np.uint8)
@@ -69,3 +70,22 @@ def decode_frame(prod, frame, dict=None, dict_huf=None, verify=0, units=0, seed=
                                   h.ctypes.data if h is not None else None, max(info.block_size, 4096),
                                   1 if (verify and info.has_checksum) else 0, units, seed, C.byref(oob))
     return list(status)[:nb], out[:total], oob.value, rv
+
+
+def decode_jobs(src, jobs, dst, block_size, dict=None, dict_huf=None, verify=0, units=0, seed=1):
+    """Run a caller-built job table (numpy structured array laid out like zxc_b200_job_t) over the source bytes `src`
+    into `dst` (uint8 ndarray, updated in place: bytes no job writes keep their value).  -> (per-job status list,
+    writes outside dst, rendezvous)"""
+    src = np.ascontiguousarray(src, np.uint8)
+    jobs = np.ascontiguousarray(jobs)
+    assert dst.flags.c_contiguous and dst.dtype == np.uint8
+    n = int(jobs.size)
+    status = (C.c_int32 * max(n, 1))()
+    oob = C.c_int(0)
+    d = np.frombuffer(dict, np.uint8) if dict else None
+    h = np.frombuffer(dict_huf, np.uint8) if dict_huf is not None else None
+    rv = lib().simt_decode_blocks(src.ctypes.data, src.size, dst.ctypes.data, dst.size, jobs.ctypes.data, n, status,
+                                  d.ctypes.data if d is not None else None, d.size if d is not None else 0,
+                                  h.ctypes.data if h is not None else None, block_size, 1 if verify else 0, units, seed,
+                                  C.byref(oob))
+    return list(status)[:n], oob.value, rv
